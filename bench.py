@@ -11,6 +11,7 @@ ncclAllGather per step INSIDE the library (hhg_plan_topk; no torch.topk / torch.
     python bench.py --gpus N --steps K --warmup W            (driver; torchrun for N > 1)
     python bench.py --impl reference ...                      (the reference's AVX2 Viterbi on the host cores)
     python bench.py --no-extras                               (skip the configs[2..4] sections)
+    python bench.py --dump-outputs bench_outputs              (also write the last timed step's results as .npy)
 
 value  : whole-job GCUPS, database resident in HBM, device-timed (CUDA events, max over ranks)
 e2e    : the same through the host-buffer C-ABI calls (hhg_query_set + hhg_viterbi_search + hhg_plan_topk): per step
@@ -59,7 +60,11 @@ def parse_args():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the configs[2..4] sections")
     ap.add_argument("--no-prefilter", action="store_true", help="(kept for old command lines; same as --no-extras)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed to DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 # ----------------------------------------------------------------------------------------------- host facts
@@ -356,6 +361,29 @@ def verify_sample(hh, qprof, db_h, hits, paths, k=16, seed=7):
     return ok
 
 
+def dump_outputs(d, merged, hits, paths, n_paths=1024, seed=11):
+    """The results of the last timed step as float64 .npy files, so that two builds can be compared output for output:
+    the merged top-K records (topk_*), every target's hit record (hits_*) and the backtrace paths of a fixed, seeded
+    sample of targets (path_targets, path_len, path_states: the states of the sampled paths, concatenated).
+    With several GPUs the hit records and paths are rank 0's shard.  About 7 MB at the headline size, mostly the
+    100,000 hit records."""
+    os.makedirs(d, exist_ok=True)
+    f64 = lambda a: np.ascontiguousarray(a, np.float64)  # noqa: E731  (exact for the int32 and float32 fields)
+    np.save(os.path.join(d, "topk_target.npy"), f64(merged["target"]))
+    for f in merged.dtype["hit"].names:
+        if f != "path_off":              # an offset into the library's own path buffer, not a result
+            np.save(os.path.join(d, f"topk_{f}.npy"), f64(merged["hit"][f]))
+    for f in hits.dtype.names:
+        if f != "path_off":
+            np.save(os.path.join(d, f"hits_{f}.npy"), f64(hits[f]))
+    pick = np.sort(np.random.default_rng(seed).choice(len(hits), min(n_paths, len(hits)), replace=False))
+    ns = hits["nsteps"][pick].astype(np.int64)
+    st = [paths[int(o):int(o) + int(k)] for o, k in zip(hits["path_off"][pick], ns)]
+    np.save(os.path.join(d, "path_targets.npy"), f64(pick))
+    np.save(os.path.join(d, "path_len.npy"), f64(ns))
+    np.save(os.path.join(d, "path_states.npy"), f64(np.concatenate(st) if st else np.zeros(0)))
+
+
 # ----------------------------------------------------------------------------------------------- extras
 def subset_db(base, idx):
     """prepared_db dict holding base targets idx[0], idx[1], ... (repeats allowed)."""
@@ -648,6 +676,8 @@ def main():
     if world == 1 and not np.array_equal(merged["target"], gids[order]):
         raise SystemExit("bench verification FAILED: device top-K differs from the host sort")
     verified += len(own)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, merged, hits, paths)
 
     # ---- per-kernel roofline figure (forward kernel timed alone with CUDA events on the same stream)
     kt = [plan.run_timed() for _ in range(3)]
@@ -693,7 +723,7 @@ def main():
     d2h = hits_pin.nbytes + int(hits_pin["nsteps"].sum()) + TOPK * 56 * world
     if world > 1:
         dist.barrier()
-    e2e_steps = max(2, min(args.steps, 5))
+    e2e_steps = args.steps
     t0 = time.perf_counter()
     for _ in range(e2e_steps):
         e2e_step()

@@ -388,6 +388,11 @@ class RefShim:
         ptr = self.lib.hhref_crf_text(C.byref(n))
         return C.string_at(ptr, n.value)
 
+    def set_contxt(self, path):
+        """par.clusterfile (-contxt): the .crf library of the following crf_state / context_pc calls."""
+        self.lib.hhref_set_contxt.argtypes = [C.c_char_p]
+        return self.lib.hhref_set_contxt(path.encode())
+
     def crf_state(self, k):
         pc = np.zeros(20, np.float64); w = np.zeros(13 * 20, np.float64); b = C.c_double()
         self.lib.hhref_crf_state.argtypes = [C.c_int, C.c_void_p, C.POINTER(C.c_double), C.c_void_p]

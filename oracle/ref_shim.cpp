@@ -795,7 +795,15 @@ static void ensure_context() {
                                g->pc_prefilter_context_engine, g->pc_prefilter_context_mode);
 }
 
-// state k of the embedded context_data.crf: pc[20], bias, w[13*20]
+// par.clusterfile (-contxt <file>): rebuild the CRF engines from that .crf file instead of the embedded context_data.crf
+extern "C" int hhref_set_contxt(const char* path) {
+  g->par->clusterfile = path;
+  InitializePseudocountsEngine(*g->par, g->context_lib, g->crf, g->pc_hhm_context_engine, g->pc_hhm_context_mode,
+                               g->pc_prefilter_context_engine, g->pc_prefilter_context_mode);
+  return g->crf ? (int)g->crf->size() : -1;
+}
+
+// state k of the CRF library in use: pc[20], bias, w[13*20]
 extern "C" int hhref_crf_state(int k, double* pc, double* bias, double* w) {
   ensure_context();
   if (!g->crf || k < 0 || k >= (int)g->crf->size()) return -1;

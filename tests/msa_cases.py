@@ -26,9 +26,8 @@ TINY = [b">master\nZ-iwHkv\n", b"#NAME some description\n>master\nlKV\n", b">ss_
 def texts():
     from hhsuite_b200 import synth
     out = [synth.a3m_text(L, n, seed, **kw).encode() for (L, n, seed, kw) in CASES]
-    q = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "oracle", "_ref", "data", "query.a3m")
-    if os.path.exists(q):
-        out.append(open(q, "rb").read())
+    from tests.util import ref_data
+    out.append(ref_data("query.a3m"))
     return out
 
 

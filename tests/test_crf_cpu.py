@@ -4,7 +4,7 @@ The context scores the CUDA kernel produces are restated here with numpy in the 
 import numpy as np
 import pytest
 
-from tests.util import bits
+from tests.util import CRF_SAMPLE, bits, ref_data, ref_data_path
 
 
 def _scores(crf, f, neff_m):
@@ -28,13 +28,14 @@ def _scores(crf, f, neff_m):
 
 def test_crf_parser_and_tail_equal_reference(refshim):
     from hhsuite_b200 import capi, synth
-    crf = capi.Crf(None, refshim.crf_text())
-    assert (crf.n_states, crf.window) == (4000, 13)
+    crf = capi.Crf(None, ref_data(CRF_SAMPLE))
+    assert refshim.set_contxt(ref_data_path(CRF_SAMPLE)) == 100
+    assert (crf.n_states, crf.window) == (100, 13)
     pc = crf.pc()
-    for k in (0, 1, 999, 3999):
+    for k in (0, 1, 50, 99):
         n, rpc, rb, rw = refshim.crf_state(k)
         w, b = crf.state(k)
-        assert n == 4000 and b == rb and np.array_equal(w.view(np.uint64), rw.view(np.uint64))
+        assert n == 100 and b == rb and np.array_equal(w.view(np.uint64), rw.view(np.uint64))
         assert np.array_equal(pc[k].view(np.uint64), rpc.view(np.uint64))       # long-double sum + log of UpdatePseudocounts
     rng = np.random.default_rng(3)
     L = 24

@@ -7,13 +7,14 @@ import numpy as np
 import pytest
 
 from tests import msa_cases
-from tests.util import bits
+from tests.util import CRF_SAMPLE, bits, ref_data, ref_data_path
 
 pytestmark = pytest.mark.gpu
 
 
 def test_context_pseudocounts_equal_reference(hhg, gpu_ctx, refshim, tmp_path):
-    crf = hhg.capi.Crf(gpu_ctx, refshim.crf_text())
+    crf = hhg.capi.Crf(gpu_ctx, ref_data(CRF_SAMPLE))
+    assert refshim.set_contxt(ref_data_path(CRF_SAMPLE)) == crf.n_states
     pb = refshim.pb()
     texts = msa_cases.texts()
     for k in (0, 2, 9, len(texts) - 1):                     # incl. the query alignment of the reference's data set
@@ -35,7 +36,8 @@ def test_default_hhblits_query_path(hhg, gpu_ctx, refshim, tmp_path):
     path = tmp_path / "q.a3m"
     path.write_bytes(qa)
     raw = hhg.capi.msa_to_hmm(gpu_ctx, qa, refshim.pb())
-    crf = hhg.capi.Crf(gpu_ctx, refshim.crf_text())
+    crf = hhg.capi.Crf(gpu_ctx, ref_data(CRF_SAMPLE))
+    assert refshim.set_contxt(ref_data_path(CRF_SAMPLE)) == crf.n_states
     p, pav = crf.pseudocounts(raw["f"], raw["neff_m"], raw["neff_hmm"], refshim.pb(), hhg.capi.Admix.hhm())
     ref = refshim.msa_to_hmm(str(path))
     ref_p, ref_pav = refshim.context_pc(ref["f"], ref["neff_m"], ref["neff_hmm"], engine=0)

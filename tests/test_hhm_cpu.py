@@ -61,12 +61,8 @@ def test_oracle_prepare_equals_compiled_reference(oracle, refshim, tmp_path, see
 
 
 def _query_path():
-    import os
-    from tests.util import ROOT
-    for p in (os.path.join(ROOT, "oracle", "_ref", "data", "query.hhm"), "/root/reference/data/query.hhm"):
-        if os.path.exists(p):
-            return p
-    pytest.skip("data/query.hhm not available")
+    from tests.util import ref_data_path
+    return ref_data_path("query.hhm")
 
 
 def test_product_tokeniser_equals_oracle(oracle):

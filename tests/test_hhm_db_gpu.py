@@ -7,7 +7,7 @@ import os
 import numpy as np
 import pytest
 
-from tests.util import ROOT, bits, golden
+from tests.util import ROOT, bits, golden, ref_data_path
 
 pytestmark = pytest.mark.gpu
 
@@ -83,9 +83,7 @@ def test_loaded_records_equal_oracle_and_goldens(hhg, gpu_ctx, oracle):
 
 def test_loaded_records_equal_compiled_reference(hhg, gpu_ctx, refshim, tmp_path):
     G = golden()
-    qpath = os.path.join(ROOT, "oracle", "_ref", "data", "query.hhm")
-    if not os.path.exists(qpath):
-        pytest.skip("oracle/_ref/data/query.hhm not shipped")
+    qpath = ref_data_path("query.hhm")
     refshim.load_query_hhm(qpath)
     texts = _texts(G, extra_seed=1, n_extra=5) + [open(qpath, "rb").read()]
     data, off, ln = _pack(texts)
@@ -205,8 +203,7 @@ def test_query_from_hhm_equals_reference_prepare_query(hhg, gpu_ctx, refshim, tm
     """hhg_query_from_hhm = HMM::Read + PrepareQueryHMM with par.nocontxt (src/hhfunc.cpp:121-160): p (all rows incl. 0
     and L+1), the complete transition rows, ss, pav and Neff_HMM bit-identical to the reference's query."""
     from hhsuite_b200 import synth
-    import os
-    cases = [os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "oracle", "_ref", "data", "query.hhm")]
+    cases = [ref_data_path("query.hhm")]
     for k, (L, ss) in enumerate([(1, False), (57, True), (300, False)]):
         f = tmp_path / f"q{k}.hhm"
         f.write_text(synth.hhm_text(L, 70 + k, f"q{k}", with_ss=ss))
@@ -230,9 +227,7 @@ def test_every_pseudocount_mode_equals_compiled_reference(hhg, gpu_ctx, refshim,
     """HMM::AddAminoAcidPseudocounts modes 0..3 (src/hhhmm.cpp:1874-1921) incl. mode 2 with pcc != 1, whose pow() is the C
     library's powf (tau computed per column on the host with the same libm) and the constant-diversity mode 3."""
     G = golden()
-    qpath = os.path.join(ROOT, "oracle", "_ref", "data", "query.hhm")
-    if not os.path.exists(qpath):
-        pytest.skip("oracle/_ref/data/query.hhm not shipped")
+    qpath = ref_data_path("query.hhm")
     refshim.load_query_hhm(qpath)
     texts = _texts(G, extra_seed=2, n_extra=4)
     data, off, ln = _pack(texts)

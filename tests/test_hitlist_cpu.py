@@ -110,11 +110,8 @@ def test_cs219_library_parser_matches_reference(refshim):
     """hhg_cs219_parse (Prefilter ctor: ContextLibrary read + TransformToLin, src/hhprefilter.cpp:28-47) on the
     reference's own cs219.lib: every float equal to what the compiled reference holds and to the golden copy."""
     import hhsuite_b200 as hh
-    from tests.util import golden
-    path = "/root/reference/data/cs219.lib"
-    if not os.path.exists(path):
-        pytest.skip("the reference's data/cs219.lib is only present in the authoring container")
-    lib = hh.capi.cs219_parse(open(path, "rb").read())
+    from tests.util import golden, ref_data
+    lib = hh.capi.cs219_parse(ref_data("cs219.lib"))
     assert lib.shape == (219, 20)
     assert np.array_equal(lib.view(np.uint32), refshim.cs219().view(np.uint32))
     assert np.array_equal(lib.view(np.uint32), np.ascontiguousarray(golden()["cs219_lin"], np.float32).view(np.uint32))

@@ -90,7 +90,9 @@ def test_emulated_filter_options_and_global_weights(emul, refshim, tmp_path, fil
 def test_emulated_context_score_kernel(emul, refshim):
     """k_crf_scores on the CPU emulator + the library's host tail == the compiled reference's CRF pseudocounts."""
     from hhsuite_b200 import capi
-    crf = capi.Crf(None, refshim.crf_text())
+    from tests.util import CRF_SAMPLE, ref_data, ref_data_path
+    crf = capi.Crf(None, ref_data(CRF_SAMPLE))
+    assert refshim.set_contxt(ref_data_path(CRF_SAMPLE)) == crf.n_states
     K, W = crf.n_states, crf.window
     Wt = np.zeros((W, 20, K)); bias = np.zeros(K)
     for k in range(K):

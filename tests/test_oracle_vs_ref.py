@@ -39,7 +39,8 @@ def test_restatement_equals_reference_kernel(oracle, refshim, seed):
 def test_synthetic_hhm_text_roundtrip_through_reference_reader(refshim, tmp_path):
     """The synthetic HHM text is accepted by HMM::Read and PrepareTemplateHMM gives finite DP inputs."""
     from hhsuite_b200 import synth
-    refshim.load_query_hhm("/root/reference/data/query.hhm")
+    from tests.util import ref_data_path
+    refshim.load_query_hhm(ref_data_path("query.hhm"))
     f = tmp_path / "s.hhm"
     f.write_text(synth.hhm_text(77, 5, "s77", with_ss=True))
     t = refshim.prepare_template_hhm(str(f))

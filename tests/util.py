@@ -1,5 +1,9 @@
 """Shared helpers for the tests (not product code)."""
+import atexit
+import gzip
 import os
+import shutil
+import tempfile
 
 import numpy as np
 
@@ -8,6 +12,32 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 def golden():
     return np.load(os.path.join(ROOT, "tests", "golden", "golden_v1.npz"))
+
+
+# every 40th state of HH-suite's data/context_data.crf (4000 states, 7 MB): a CRF library small enough to store
+CRF_SAMPLE = "context_data_every40.crf"
+
+
+def ref_data(name):
+    """Bytes of a file of HH-suite's data/ directory (query.hhm, query.a3m, cs219.lib, CRF_SAMPLE; stored gzipped)."""
+    with gzip.open(os.path.join(ROOT, "tests", "golden", "data", name + ".gz"), "rb") as f:
+        return f.read()
+
+
+_ref_dir = None
+
+
+def ref_data_path(name):
+    """Path of an uncompressed copy of ref_data(name) in a temporary directory of this process."""
+    global _ref_dir
+    if _ref_dir is None:
+        _ref_dir = tempfile.mkdtemp(prefix="hhg_refdata_")
+        atexit.register(shutil.rmtree, _ref_dir, True)
+    path = os.path.join(_ref_dir, name)
+    if not os.path.exists(path):
+        with open(path, "wb") as f:
+            f.write(ref_data(name))
+    return path
 
 
 def bits(x):
