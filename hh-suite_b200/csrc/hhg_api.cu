@@ -356,6 +356,13 @@ static int pack_profiles(hhg_ctx* ctx, int n, const int32_t* L, const int64_t* p
       memcpy(htr.data() + to[k], tr + tr_off[t0 + k], (size_t)(LL[k] + 1) * 7 * sizeof(float));
       if (ss) memcpy(hss.data() + so[k], ss + ss_off[t0 + k], (size_t)(LL[k] + 2));
     }
+    // emissions are probabilities (ratios): the forward kernel's dot product relies on them being >= 0 (-0.0 is fine)
+    for (int k = 0; k < m; ++k) {
+      const float* row = hp.data() + po[k] + 20;
+      for (int a = 0; a < LL[k] * 20; ++a)
+        if (row[a] < 0.0f)
+          return fail(HHG_EINVAL, "profile %d: emission %g at column %d is negative", t0 + k, row[a], a / 20 + 1);
+    }
     const long long cols = (t1 < n ? col_off[t1] : total_cols) - col_off[t0];
     CK(dp.ensure(np)); CK(dtr.ensure(ntr)); CK(dL.ensure(m)); CK(dcol.ensure(m)); CK(dpo.ensure(m));
     CK(dto.ensure(m)); CK(dso.ensure(m));

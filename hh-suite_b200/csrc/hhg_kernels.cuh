@@ -150,7 +150,9 @@ __device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
       "r"(parity)
       : "memory");
 }
-// log2f4 (src/hhutil-inl.h:509-541), degree-4 minimax, unfused.  x >= 0.
+// log2f4 (src/hhutil-inl.h:509-541), degree-4 minimax, unfused.  The sign bit of x must be clear: the reference
+// masks it off (i & 0x7F800000), this version does not (ptxas folds the shift and the OR below into one LEA.HI;
+// a mask costs an instruction per cell).  dot20_dev never returns a value with the sign bit set.
 // The exponent int->float conversion uses the exact magic-number form (no I2F on the hot path):
 // bits(8388608.0f) + eb is the float 8388608+eb; subtracting 8388735 (=2^23+127) is exact.
 __device__ __forceinline__ float log2f4_dev(float x) {
@@ -205,7 +207,9 @@ __device__ __forceinline__ float dot20_dev(const unsigned long long (&t)[10], co
   float r0, r1, r2, r3;
   unpack2(a01, r0, r1);
   unpack2(a23, r2, r3);
-  return __fadd_rn(__fadd_rn(r0, r1), __fadd_rn(r2, r3));
+  // |.| on both halves (free FADD operand modifiers): emissions are >= 0 (the C-ABI refuses negative ones), so this
+  // changes only a -0.0 sum, from columns of -0.0 emissions, into +0.0, where the reference's log2f4 gives -127
+  return __fadd_rn(fabsf(__fadd_rn(r0, r1)), fabsf(__fadd_rn(r2, r3)));
 }
 
 // one 16-byte operand of the job-interleaved stream: L2-only load (a line is read once per strip and SM; an L2
